@@ -16,18 +16,26 @@ second = CHAINS*ITERS*5 / time.
               interpreter; the JVM reference cannot run here) on the box's host cores, bounded sample.
 
 Multi-GPU (torchrun): chains are sharded over ranks, no data-path collective, weak scaling (CHAINS per GPU fixed).
+
+--dump-outputs DIR writes the draws of the last timed step (a seeded sample of them, see dump_outputs) so that two builds
+can be compared output for output: the seeds, and therefore the inputs, are the same in every run with the same arguments.
+The bench writes nothing into the source tree: kernels compiled at run time are cached in a temporary directory.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only; no __pycache__ in it either way
 
 import numpy as np  # noqa: E402
 
@@ -35,6 +43,8 @@ N_DIM = 10
 N_STEPS = 5
 STEP_SIZE = 0.1
 METRIC = "leapfrog_steps_x_chains_per_sec"
+DUMP_LAST_DRAW_BYTES = 16_000_000  # --dump-outputs writes less than 64 MB in all
+DUMP_SAMPLES_BYTES = 47_000_000
 
 
 def bytes_per_leapfrog_step(n, L):
@@ -352,6 +362,28 @@ def extra_configs(args, torch, dist, api, abi, rank, local_rank, world):
     return out
 
 
+def _seeded_chains(total, k):
+    """all chains when k covers them, else a fixed, seeded choice of k of them (ascending)"""
+    if k >= total:
+        return np.arange(total)
+    return np.sort(np.random.default_rng(0).choice(total, k, replace=False))
+
+
+def dump_outputs(out_dir, d_samples):
+    """The draws the last timed step returned to its caller (d_samples: [iterations][n][chains] fp64 on the device), as
+      last_draw.npy  [n][chains]          the final position of every chain (a seeded sample beyond 16 MB)
+      samples.npy    [iterations][n][k]   every draw of a seeded sample of k chains (at most 47 MB; the last
+                                          iterations only if one chain's draws alone exceed that)"""
+    import torch
+    iters, n, chains = d_samples.shape
+    os.makedirs(out_dir, exist_ok=True)
+    pick = torch.from_numpy(_seeded_chains(chains, DUMP_LAST_DRAW_BYTES // (8 * n))).to(d_samples.device)
+    np.save(os.path.join(out_dir, "last_draw.npy"), d_samples[-1].index_select(1, pick).cpu().numpy())
+    it = min(iters, DUMP_SAMPLES_BYTES // (8 * n))
+    pick = torch.from_numpy(_seeded_chains(chains, DUMP_SAMPLES_BYTES // (8 * n * it))).to(d_samples.device)
+    np.save(os.path.join(out_dir, "samples.npy"), d_samples[iters - it:].index_select(2, pick).cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -365,7 +397,11 @@ def main():
     ap.add_argument("--grad", default="auto", choices=["auto", "symbolic", "adjoint"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the cfg3/cfg4/cfg5 side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the draws of the last timed step to DIR/*.npy (rank 0's chains when sharded)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -377,7 +413,12 @@ def main():
     from rainier_b200 import abi, api
 
     if "RN_KERNEL_CACHE" not in os.environ and os.path.isdir(os.path.join(ROOT, "build", "kcache")):
-        os.environ["RN_KERNEL_CACHE"] = os.path.join(ROOT, "build", "kcache")  # NVRTC of the 1000-parameter model: ~35 s otherwise
+        # NVRTC of the 1000-parameter model: ~35 s otherwise.  A temporary copy of build()'s cubins takes the kernels
+        # compiled at run time, so that the tree stays as build() left it
+        kcache = tempfile.mkdtemp(prefix="rn_kcache_")
+        atexit.register(shutil.rmtree, kcache, True)
+        shutil.copytree(os.path.join(ROOT, "build", "kcache"), kcache, dirs_exist_ok=True)
+        os.environ["RN_KERNEL_CACHE"] = kcache
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -432,6 +473,8 @@ def main():
     total_steps = float(world) * C_ * I_ * N_STEPS * args.steps
     value = total_steps / (ms_max * 1e-3)
     smp.close()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_samples)
 
     # ---------------- end-to-end leg: public one-call API (rn_sample over the C ABI), HOST buffers ----------------
     # every step: seeds host->device, all samples device->host.  Headline = page-locked caller buffer (rn_host_alloc,
@@ -469,7 +512,7 @@ def main():
         units = float(world) * C_ * I_ * N_STEPS
         return units / med, {"median": med * 1e3, "min": lo * 1e3, "mean": mean * 1e3, "max": hi * 1e3}
 
-    n_e2e = max(3, min(args.steps, 10))
+    n_e2e = args.steps
     # supplementary: the same call returning only Trace.diagnostics (rHat / ESS reduced on the device, rn_config.diagnostics
     # with samples == NULL) -- what the path does when the caller needs summaries rather than 1.2 GB of draws
     diag_cfg, keep2 = api.lower_config(cfg)
