@@ -70,10 +70,8 @@ struct Emitter {
   }
 
   // see row_body(): splits the row statements into independent dataflow components and merges them round-robin
-  // `fused` (optional): ONE order in which every group of components runs its forward statements and then, at once, its reverse
-  // statements -- see row_body()
   void interleave_components(const TargetInfo& T, const std::set<int>& body, std::vector<int>& order_fwd,
-                             std::vector<int>& order_bwd, std::vector<int>* fused = nullptr) const {
+                             std::vector<int>& order_bwd) const {
     const int BIG = 4;  // two components of at least this many statements meeting in one statement = a joiner
     std::map<int, int> parent, size;  // union-find over statement ids
     std::set<int> tail;
@@ -85,43 +83,11 @@ struct Emitter {
       return x;
     };
     std::vector<int> ops;
-    // fused mode: the additions that only fold the row's terms into the accumulated value (reachable from an accumulate statement
-    // through single-use ADD nodes) are joiners by definition -- otherwise the running sum swallows every observation it meets
-    // while that observation's component is still small, and the whole row becomes one chain
-    std::set<int> fold;
-    if (fused) {
-      std::map<int, int> uses;
-      auto count_ops = [&](int s) {
-        operands(s, ops);
-        for (int o : ops) uses[o]++;
-      };
-      for (int id : T.row_fwd)
-        if (body.count(id)) count_ops(id);
-      for (int id : T.row_bwd)
-        if (body.count(id)) count_ops(id);
-      for (const AccStmt& a : T.row_acc) uses[a.node] += 2;  // (roots: entered below whatever their count)
-      for (const ScatterStmt& sc : T.row_scatter) uses[sc.node] += 2, uses[sc.index_node] += 2;
-      std::vector<int> stack;
-      for (const AccStmt& a : T.row_acc)
-        if (body.count(a.node)) stack.push_back(a.node);
-      std::set<int> roots(stack.begin(), stack.end());
-      while (!stack.empty()) {
-        const int id = stack.back();
-        stack.pop_back();
-        const Node& n = P.nodes[id];
-        if (n.kind != K_BINARY || n.op != RIR_B_ADD) continue;
-        if (!roots.count(id) && uses[id] != 1) continue;
-        if (!fold.insert(id).second) continue;
-        if (body.count(n.a)) stack.push_back(n.a);
-        if (body.count(n.b)) stack.push_back(n.b);
-      }
-    }
     auto classify = [&](int s) {
       operands(s, ops);
-      bool is_tail = fold.count(s) > 0;
+      bool is_tail = false;
       std::set<int> comps;
       for (int o : ops) {
-        if (is_tail) break;
         if (!body.count(o)) continue;
         if (tail.count(o)) {
           is_tail = true;
@@ -190,77 +156,6 @@ struct Emitter {
         }
       out.insert(out.end(), tails.begin(), tails.end());
     };
-    if (fused) {
-      std::vector<int> comp_order, tails_f, tails_b;
-      std::map<int, std::vector<int>> lf, lb;
-      for (int id : fwd) {
-        if (tail.count(id)) {
-          tails_f.push_back(id);
-          continue;
-        }
-        const int c = find(id);
-        if (!lf.count(c) && !lb.count(c)) comp_order.push_back(c);
-        lf[c].push_back(id);
-      }
-      for (int id : bwd) {
-        if (tail.count(id)) {
-          tails_b.push_back(id);
-          continue;
-        }
-        const int c = find(id);
-        if (!lf.count(c) && !lb.count(c)) comp_order.push_back(c);
-        lb[c].push_back(id);
-      }
-      const size_t W = (size_t)std::max(1, opt.interleave);
-      auto rr = [&](std::map<int, std::vector<int>>& lists, size_t g0) {
-        std::vector<size_t> pos(W, 0);
-        for (bool any = true; any;) {
-          any = false;
-          for (size_t k = g0; k < std::min(comp_order.size(), g0 + W); k++) {
-            const std::vector<int>& l = lists[comp_order[k]];
-            if (pos[k - g0] < l.size()) {
-              fused->push_back(l[pos[k - g0]++]);
-              any = true;
-            }
-          }
-        }
-      };
-      // joiners are issued as soon as their operands exist (a fold addition right after the term it adds), not at the end
-      std::vector<int> pending(tails_f);
-      pending.insert(pending.end(), tails_b.begin(), tails_b.end());
-      std::set<int> done;
-      size_t flushed = 0;
-      auto flush = [&]() {
-        for (size_t i = flushed; i < fused->size(); i++) done.insert((*fused)[i]);
-        for (bool any = true; any;) {
-          any = false;
-          for (size_t i = 0; i < pending.size(); i++) {
-            const int t = pending[i];
-            if (t < 0) continue;
-            operands(t, ops);
-            bool ready = true;
-            for (int o : ops)
-              if (body.count(o) && !done.count(o)) ready = false;
-            if (!ready) continue;
-            fused->push_back(t);
-            done.insert(t);
-            pending[i] = -1;
-            any = true;
-          }
-        }
-        flushed = fused->size();
-      };
-      for (size_t g0 = 0; g0 < comp_order.size(); g0 += W) {
-        rr(lf, g0);
-        flush();
-        rr(lb, g0);
-        flush();
-      }
-      flush();
-      for (int t : pending)
-        if (t >= 0) fused->push_back(t);  // (cannot happen for an acyclic body; keeps the order total)
-      return;
-    }
     schedule(fwd, order_fwd);
     schedule(bwd, order_bwd);
   }
@@ -301,15 +196,10 @@ struct Emitter {
     auto emit_acc = [&](const AccStmt& a) { os << ind << accref(a.slot) << " += " << val(a.node) << ";\n"; };
     auto emit_scatter = [&](const ScatterStmt& sc) {
       if (atomic_scatter) {
-        auto ri = row_index.find(sc.index_node);
-        if (ri != row_index.end() && ri->second.low == sc.low && ri->second.len == sc.len) {
-          // the forward Lookup's index (-1: outside the table, flag already raised there)
-          os << ind << "{ const int k = " << ri->second.var << "; const bool bad = k < 0; rn_scatter_add(&scr["
-             << (scatter_base_off + smem_slot[sc.slot_base]) << " + (bad ? 0 : k)], bad ? 0.0 : " << val(sc.node) << "); }\n";
-          return;
-        }
         // branch-free (an index outside the table raises the flag and adds 0 to entry 0) and in the shared state space: the
-        // generic atomicAdd carries one code path per address space behind a run-time test, 16 times per row body on cfg 5
+        // generic atomicAdd carries one code path per address space behind a run-time test, 16 times per row body on cfg 5.
+        // The index is converted again rather than kept from the forward Lookup: reusing it lost 3 % on cfg 5 (2.455e5 -> 2.374e5,
+        // profiles/r2_bench_row_libm_ab_v2.txt) -- eight more values live across the reverse sweep's fence at 128 registers
         os << ind << "{ const int k = rn_d2i(" << val(sc.index_node) << ") - (" << sc.low << "); const bool bad = (unsigned)k >= " << sc.len
            << "u; err |= (int)bad; rn_scatter_add(&scr[" << (scatter_base_off + smem_slot[sc.slot_base]) << " + (bad ? 0 : k)], bad ? 0.0 : "
            << val(sc.node) << "); }\n";
@@ -329,8 +219,7 @@ struct Emitter {
       auto is = sc_at.find(id);
       if (is != sc_at.end())
         for (const ScatterStmt* sc : is->second) {
-          auto ri = row_index.find(sc->index_node);
-          if (!(atomic_scatter && ri != row_index.end() && ri->second.low == sc->low && ri->second.len == sc->len)) need_col(sc->index_node);
+          need_col(sc->index_node);
           emit_scatter(*sc);
         }
     };
@@ -338,39 +227,12 @@ struct Emitter {
     // results only meet in a final sum.  Emitting them one after the other leaves each warp with a single serial
     // dependency chain (a 50-term dot product is 50 dependent FMAs; ncu: stall_wait dominates at 8 warps/SM), so the
     // statements of the components are interleaved round-robin; "joiner" statements (and everything downstream of
-    // them) follow in their original order.  Values are unchanged (SSA); only the issue order moves.
+    // them) follow in their original order.  Values are unchanged (SSA); only the issue order moves.  The reverse sweep
+    // follows the forward sweep of the whole row: issuing a group's reverse statements right after its forward statements
+    // (no second read of the tile) measured cfg 5 -10 %, cfg 2s and rows-across-lanes cfg 3 +1 % (profiles/r2_bench_fused_sweeps_ab_v1.txt).
     std::vector<int> order_fwd, order_bwd;
-    // RN_ROW_FUSED_SWEEPS (warp-per-chain, experiment switch): the reverse statements of a group of observations follow its forward
-    // statements directly instead of after the forward sweep of the whole row.  A component's reverse statements read only its own
-    // forward values (anything that reads a joiner is a joiner itself and stays at the end), so this is the same dataflow; the
-    // columns a group loaded are still in registers for its reverse sweep: no fence, no second read of the tile (ncu, cfg 5:
-    // shared-memory wavefronts are 53 % of the pipe's capacity and `short_scoreboard` the first stall reason; each column is read
-    // twice per observation today).
-    const bool fused_sweeps = wpc && getenv("RN_ROW_FUSED_SWEEPS") && atoi(getenv("RN_ROW_FUSED_SWEEPS")) != 0;
-    if (fused_sweeps) {
-      std::vector<int> order;
-      interleave_components(T, body, order_fwd, order_bwd, &order);
-      col_suffix.clear();
-      row_index.clear();
-      capture_row_index = false;
-      for (int id : order) one(id);
-      for (const AccStmt* a : acc_tail) {
-        need_col(a->node);
-        emit_acc(*a);
-      }
-      for (const ScatterStmt* sc : sc_tail) {
-        need_col(sc->index_node);
-        need_col(sc->node);
-        emit_scatter(*sc);
-      }
-      return;
-    }
     interleave_components(T, body, order_fwd, order_bwd);
     col_suffix.clear();
-    row_index.clear();
-    // opt-in: measured on B200 it LOSES 3 % on cfg 5 (2.455e5 -> 2.374e5, profiles/r2_bench_row_libm_ab_v2.txt) -- eight more values
-    // live across the reverse sweep's fence at 128 registers cost more than the second LDS + F2I they replace
-    capture_row_index = atomic_scatter && getenv("RN_SCATTER_REUSE_INDEX") && atoi(getenv("RN_SCATTER_REUSE_INDEX")) != 0;
     for (int id : order_fwd) one(id);
     if (!order_bwd.empty()) {
       os << ind << "RN_FENCE();\n";
@@ -383,14 +245,11 @@ struct Emitter {
       emit_acc(*a);
     }
     for (const ScatterStmt* sc : sc_tail) {
-      auto ri = row_index.find(sc->index_node);
-      if (!(atomic_scatter && ri != row_index.end() && ri->second.low == sc->low && ri->second.len == sc->len)) need_col(sc->index_node);
+      need_col(sc->index_node);
       need_col(sc->node);
       emit_scatter(*sc);
     }
     col_suffix.clear();
-    capture_row_index = false;
-    row_index.clear();
   }
 
   std::string acc_ref(int slot) const {
@@ -425,25 +284,19 @@ struct Emitter {
   // pow() per observation of a logistic regression
   // Row bodies of the warp-per-chain shape: total, branch-free exp / log / reciprocal (rn_prelude.cuh: rn_row_*) instead of CUDA's
   // exp(), log() and 1.0 / x, each of which ends a basic block with its range test -- and the statements of 4 or 8 observations
-  // are interleaved precisely so that ptxas can overlap their chains.  RN_ROW_LIBM=0 keeps CUDA's functions (A/B).
+  // are interleaved precisely so that ptxas can overlap their chains.
   // Measured on B200 (profiles/r2_bench_row_libm_ab_v1.txt, ..._v2.txt): the rows-across-lanes body gains -- cfg 5: 2.22e5 -> 2.46e5
   // with two observations in flight where the arguments of exp are wild (every proposal rejected far from the mode: CUDA's exp
   // takes its out-of-line completion there), 2.41e5 -> 2.46e5 after an adaptive warmup --, the chain-batched DMMA kernel loses (cfg 3: 5.25e5 -> 4.66e5; at 128 registers the four elements
-  // of its helper in one basic block spill: stack 976 -> 4776 bytes) -- so the default is on for kernels without the DMMA path
-  // and off for those with it (helper and its rows-across-lanes tail alike: that kernel stays exactly what round 2 validated).
-  // ... and neither do row bodies that keep many accumulators in registers: the rows-across-lanes form of cfg 3 (RN_MMA=0: 51
-  // accumulators) runs 5.4e4 with the row functions against 2.1e5 with CUDA's libm, the merged block spills.  The default is on
-  // only where the registers have room: no DMMA path and at most RN_ROW_LIBM_MAX_ACC (8) register accumulators (cfg 5: 2).
-  bool in_mma_helper = false, kernel_uses_mma = false;
-  int kernel_reg_accumulators = 0;
-  bool row_libm_on() const {
-    if (const char* e = getenv("RN_ROW_LIBM")) return atoi(e) != 0;
-    int max_acc = 8;
-    if (const char* e = getenv("RN_ROW_LIBM_MAX_ACC")) max_acc = atoi(e);
-    return !kernel_uses_mma && kernel_reg_accumulators <= max_acc;
-  }
+  // of its helper in one basic block spill: stack 976 -> 4776 bytes) -- so they are used in kernels without the DMMA path
+  // and not in those with it (helper and its rows-across-lanes tail alike: that kernel stays exactly what round 2 validated).
+  // ... and neither in row bodies that keep many accumulators in registers: the rows-across-lanes form of cfg 3 (RN_MMA=0: 51
+  // accumulators) runs 5.4e4 with the row functions against 2.1e5 with CUDA's libm, the merged block spills.  So they are used
+  // only where the registers have room: no DMMA path and at most 8 register accumulators (cfg 5: 2).  Set by density_wpc().
+  bool row_functions = false;
+  bool in_mma_helper = false;
   std::string recip(const std::string& x, bool row_variant) const {
-    return (row_variant && row_libm_on()) ? "rn_row_rcp(" + x + ")" : "(1.0 / " + x + ")";
+    return (row_variant && row_functions) ? "rn_row_rcp(" + x + ")" : "(1.0 / " + x + ")";
   }
   std::string pow_expr(int a, int b, bool derived, bool row_variant = false) const {
     const Node& e = P.nodes[b];
@@ -472,26 +325,13 @@ struct Emitter {
         if (c == 1.5) return "(" + x + " * sqrt(" + x + "))";
       }
     }
-    if (merged && !row_variant) return "rn_pow_m<SLOW>(" + x + ", " + val(b) + ", bad)";
     return std::string(row_variant ? "rn_pow_libm(" : "rn_pow(") + x + ", " + val(b) + ")";
   }
   bool row_libm(const Node& n) const { return wpc && (n.region == R_ROW_FWD || n.region == R_ROW_BWD); }
-  // density_tpc() of a data-free model in parity mode: the fdlibm calls of the whole density share ONE fallback branch -- the
-  // common paths accumulate a flag (rn_exp_m<0> ...), and only if it is set the density is evaluated again, out of line, by the
-  // complete functions (rn_exp_m<1> ...).  See density_tpc().
-  bool merged = false;
-  // warp-per-chain row bodies: a Lookup's table index (D2I, range test) is kept in an int and reused by the scatter-add of its
-  // adjoint in the reverse sweep, instead of re-loading the index column from the tile and converting it again (ncu, cfg 5:
-  // the F2I behind that second LDS was 9.5 % of the row loop's stall samples, all short_scoreboard).  key: index node.
-  struct RowIndex { int low, len; std::string var; };
-  std::map<int, RowIndex> row_index;
-  bool capture_row_index = false;
 
   void stmt(int id, const char* indent) {
     const Node& n = P.nodes[id];
     if (n.kind == K_CONST || n.kind == K_INPUT) return;
-    if (n.kind == K_LOOKUP && wpc && tab_off.count(id) && capture_row_index && !row_index.count(n.a))
-      os << indent << "int ki" << id << node_suffix << ";\n";
     os << indent << "const double " << val(id) << " = ";
     switch (n.kind) {
       case K_UNARY: {
@@ -502,12 +342,10 @@ struct Emitter {
           // the oracle anyway (1e-13 agreement), and fdlibm costs twice the instructions.  Everything that stays
           // bit-exact -- invariant parts, data-free targets, the thread-per-chain kernels -- keeps fdlibm.
           case RIR_U_EXP:
-            if (merged) { os << "rn_exp_m<SLOW>(" << x << ", bad)"; break; }
-            os << (row_libm(n) && !getenv("RN_ROW_EXP_FDLIBM") ? (row_libm_on() ? "rn_row_exp(" : "exp(") : "rn_exp(") << x << ")";
+            os << (row_libm(n) ? (row_functions ? "rn_row_exp(" : "exp(") : "rn_exp(") << x << ")";
             break;
           case RIR_U_LOG:
-            if (merged) { os << "rn_log_m<SLOW>(" << x << ", bad)"; break; }
-            os << (row_libm(n) ? (row_libm_on() ? "rn_row_log(" : "log(") : "rn_log(") << x << ")";
+            os << (row_libm(n) ? (row_functions ? "rn_row_log(" : "log(") : "rn_log(") << x << ")";
             break;
           case RIR_U_ABS: os << "fabs(" << x << ")"; break;
           case RIR_U_NOOP: os << x; break;
@@ -536,7 +374,7 @@ struct Emitter {
             // instructions of cfg 3 (profiles/r2_ncu_cfg3_mma_v1_regions.txt).  adj * (1 / x) keeps the inline path (the
             // numerator is 1); one more rounding, in a region that agrees with the oracle to 1e-13 by construction
             // (tree sums), not bit for bit.  Everything that is compared bit for bit keeps the exact quotient.
-            if (wpc && n.region == R_ROW_BWD && !getenv("RN_EXACT_ROW_DIV"))
+            if (wpc && n.region == R_ROW_BWD)
               os << "(" << x << " * " << recip(y, true) << ")";
             else
               os << "(" << x << " / " << y << ")";
@@ -549,12 +387,6 @@ struct Emitter {
       case K_LOOKUP: {
         // D2I ; tableswitch ; default -> throw (ir/ExprMethodGenerator.scala:50-56): flag + NaN instead of a fault
         if (wpc && tab_off.count(id)) {
-          if (capture_row_index && !row_index.count(n.a)) {
-            const std::string var = "ki" + std::to_string(id) + node_suffix;
-            row_index[n.a] = RowIndex{n.d, n.c, var};
-            os << "rn_tab_lookup_k(scr + " << tab_off.at(id) << ", " << n.c << ", " << n.d << ", " << val(n.a) << ", err, " << var << ")";
-            break;
-          }
           os << "rn_tab_lookup(scr + " << tab_off.at(id) << ", " << n.c << ", " << n.d << ", " << val(n.a) << ", err)";
           break;
         }
@@ -587,15 +419,8 @@ struct Emitter {
     os << "// ---- emitted: log-density and gradient of the frozen DAG (" << (P.symbolic ? "symbolic" : "adjoint")
        << " gradient) ----\n";
     lookup_helpers();
-    bool data_free = true;
-    for (const TargetInfo& T : P.targets) data_free = data_free && !T.streamed();
-    merged = data_free && !opt.fast_math && getenv("RN_MERGED_FALLBACK") && atoi(getenv("RN_MERGED_FALLBACK")) != 0;  // opt-in (A/B)
-    if (merged)
-      os << "template <int SLOW>\nRN_DEVICE void rn_density_t(const double (&q)[RN_N], double& dens, double (&grad)[RN_N], "
-            "const double* RN_RESTRICT data, int& err, bool& bad) {\n";
-    else
-      os << "RN_DEVICE void rn_density(const double (&q)[RN_N], double& dens, double (&grad)[RN_N], "
-            "const double* RN_RESTRICT data, int& err) {\n";
+    os << "RN_DEVICE void rn_density(const double (&q)[RN_N], double& dens, double (&grad)[RN_N], "
+          "const double* RN_RESTRICT data, int& err) {\n";
     os << "  (void)data; (void)err;\n";
     os << "  double acc[RN_NSLOTS];\n  for (int s = 0; s < RN_NSLOTS; s++) acc[s] = 0.0;\n";
     for (int id : P.inv_fwd) stmt(id, "  ");
@@ -623,16 +448,6 @@ struct Emitter {
       for (uint32_t i = 0; i < P.n_params; i++) os << "  grad[" << i << "] = " << val(P.grad_nodes[i]) << ";\n";
     }
     os << "}\n";
-    if (merged) {
-      // one straight-line instance of the common paths; the complete functions re-evaluate the density out of line when any
-      // argument left a common path (NaN / inf / subnormal / overflow candidates, |f| < 2^-20 in log, special exponents of pow)
-      // (the second instance is inlined too: an out-of-line function taking q / grad by reference would pin those arrays to
-      // local memory on the hot path -- measured in SASS: 30 STL.64 + 30 LDL.64 per leapfrog step; its libm calls are out of line)
-      os << "RN_DEVICE void rn_density(const double (&q)[RN_N], double& dens, double (&grad)[RN_N], "
-            "const double* RN_RESTRICT data, int& err) {\n  bool bad = false;\n  rn_density_t<0>(q, dens, grad, data, err, bad);\n"
-            "  if (bad) rn_density_t<1>(q, dens, grad, data, err, bad);\n}\n";
-      merged = false;
-    }
   }
 
   // Function flavour: forward evaluation of the m outputs of Compiler.compile(inputs, outputs).  An output is stored as
@@ -970,14 +785,8 @@ struct Emitter {
         os << "  const double c" << k << sfx(e) << " = rn_lds(" << (e & 1 ? "rp1" : "rp0") << ", roff + " << (e >> 1) * 8 + (local_col(T, k) - d.cmin) * pitch << ");\n";
     };
     std::vector<int> o;
-    // elements in flight per statement (RN_MMA_ELEMS, experiment switch; default 4): with the branch-free row functions all four
-    // chains sit in one basic block and ptxas overlaps them completely -- at 128 registers that can cost more in spills than it
-    // gains; 2 runs the helper's body twice over two elements
-    int EW = 4;
-    if (const char* ev = getenv("RN_MMA_ELEMS")) EW = std::max(1, std::min(4, atoi(ev)));
-    int e_lo = 0, e_hi = 4;
     auto one = [&](int id) {
-      for (int e = e_lo; e < e_hi; e++) {
+      for (int e = 0; e < 4; e++) {
         node_suffix = col_suffix = sfx(e);
         if (id == d.z) {  // the dot itself: the tensor core's sum, plus the fold's first operand
           if (d.base >= 0) {
@@ -993,30 +802,26 @@ struct Emitter {
         stmt(id, "  ");
       }
     };
-    for (e_lo = 0; e_lo < 4; e_lo += EW) {
-      e_hi = std::min(4, e_lo + EW);
-      if (e_lo > 0) os << "  RN_FENCE();\n";
-      bool z_done = false;
-      for (int id : d.fwd) {
-        one(id);
-        if (id == d.z) z_done = true;
-      }
-      if (!z_done) one(d.z);
-      for (int l : d.leaves)
-        for (int e = e_lo; e < e_hi; e++) {
-          node_suffix = col_suffix = sfx(e);
-          need_col(l, e);
-          os << "  dens += " << val(l) << ";\n";
-        }
-      for (int id : d.bwd) one(id);
-      for (int e = e_lo; e < e_hi; e++) {
+    bool z_done = false;
+    for (int id : d.fwd) {
+      one(id);
+      if (id == d.z) z_done = true;
+    }
+    if (!z_done) one(d.z);
+    for (int l : d.leaves)
+      for (int e = 0; e < 4; e++) {
         node_suffix = col_suffix = sfx(e);
-        need_col(d.w, e);
-        os << "  wout[" << e << "] = " << val(d.w) << ";\n";
-        for (const AccStmt& a : d.acc) {
-          need_col(a.node, e);
-          os << "  osum[" << a.slot << "] += " << val(a.node) << ";\n";
-        }
+        need_col(l, e);
+        os << "  dens += " << val(l) << ";\n";
+      }
+    for (int id : d.bwd) one(id);
+    for (int e = 0; e < 4; e++) {
+      node_suffix = col_suffix = sfx(e);
+      need_col(d.w, e);
+      os << "  wout[" << e << "] = " << val(d.w) << ";\n";
+      for (const AccStmt& a : d.acc) {
+        need_col(a.node, e);
+        os << "  osum[" << a.slot << "] += " << val(a.node) << ";\n";
       }
     }
     node_suffix.clear();
@@ -1665,11 +1470,10 @@ struct Emitter {
     if (!any_full) mma_all_ok = false;
     if (!mma_all_ok) mma_shared_doubles = 0;
     const bool use_mma = opt.mma && mma_all_ok;
-    kernel_uses_mma = use_mma;
     int n_reg_acc = 0;
     for (int sl = 0; sl < P.n_slots; sl++)
       if (smem_slot[sl] < 0) n_reg_acc++;
-    kernel_reg_accumulators = n_reg_acc;
+    row_functions = !use_mma && n_reg_acc <= 8;
     rr_plan();
     // cross-warp reduction scratch of the chain's group (K warps): [warp][register accumulators..., err]; the sums of the
     // re-rolled families go through it too, before and after the row loops
@@ -1681,9 +1485,6 @@ struct Emitter {
     os << "#define RN_WPC_RED_OFF " << red_off << "\n";
     os << "RN_DEVICE double rn_tab_lookup(const double* tab, int len, int low, double idx, int& err) {\n"
           "  const int k = rn_d2i(idx) - low;\n  const bool bad = (unsigned)k >= (unsigned)len;\n  err |= (int)bad;\n"
-          "  const double v = tab[bad ? 0 : k];\n  return bad ? RN_NAN : v;\n}\n";
-    os << "RN_DEVICE double rn_tab_lookup_k(const double* tab, int len, int low, double idx, int& err, int& kout) {\n"
-          "  const int k = rn_d2i(idx) - low;\n  const bool bad = (unsigned)k >= (unsigned)len;\n  err |= (int)bad;\n  kout = bad ? -1 : k;\n"
           "  const double v = tab[bad ? 0 : k];\n  return bad ? RN_NAN : v;\n}\n";
     os << "RN_DEVICE double rn_warp_sum(double x) {\n  RN_UNROLL\n  for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);\n  return x;\n}\n";
     lookup_helpers();
@@ -1823,7 +1624,7 @@ WpcSizes wpc_sizes(const Program& P, const EmitOptions& opt) {
       z.tile_doubles = std::max(z.tile_doubles, (int)T.n_cols * opt.pitch((size_t)(&T - &P.targets[0])) * std::max(1, opt.wpc_k));
   z.mma_ok = E.mma_all_ok;
   z.mma_shared_doubles = E.mma_shared_doubles;
-  z.reg_accumulators = E.kernel_reg_accumulators;
+  z.row_functions = E.row_functions;
   return z;
 }
 

@@ -47,7 +47,7 @@ struct WpcSizes {
   int tile_doubles = 0;
   bool mma_ok = false;       // every streamed target with full tiles can take the chain-batched DMMA path
   int mma_shared_doubles = 0;  // CTA-shared doubles of that path: 8 per-warp column-block regions + the reduction scratch
-  int reg_accumulators = 0;    // accumulators the row bodies keep in registers (decides the row functions' default, see rn_emit.cpp)
+  bool row_functions = false;  // the row bodies use the branch-free rn_row_* functions instead of CUDA's libm (rule: rn_emit.cpp)
 };
 WpcSizes wpc_sizes(const Program& P, const EmitOptions& opt);
 

@@ -27,7 +27,6 @@
 #include <map>
 #include <memory>
 #include <mutex>
-#include <sstream>
 #include <string>
 #include <thread>
 #include <tuple>
@@ -289,7 +288,7 @@ extern "C" const char* rn_version(void);
 // source_only: just emit (rn_emit_source, the analogue of rainier-decompile) -- no NVRTC run, nothing cached
 static int get_kernel(rn_model* m, const rn_config* cfg, Kernel** out, std::string* source_only = nullptr, size_t chains_hint = 0) {
   KernelKey key = key_for(m, cfg);
-  if (key.backend == 0 && chains_hint > 0 && !(getenv("RN_GENERIC_BLOCK") && atoi(getenv("RN_GENERIC_BLOCK")) != 0)) key.block = (int)tpc_block_for(chains_hint);
+  if (key.backend == 0 && chains_hint > 0) key.block = (int)tpc_block_for(chains_hint);
   auto it = m->kernels.find(key);
   if (it != m->kernels.end()) {
     if (source_only)
@@ -394,10 +393,7 @@ static int get_kernel(rn_model* m, const rn_config* cfg, Kernel** out, std::stri
     // (with the branch-free row functions the components in flight share ONE basic block and ptxas overlaps them completely:
     // two at 128 registers -- cfg 5: 2.46e5 against 2.41e5 with four, profiles/r2_bench_row_libm_ab_v1.txt; the DMMA kernels
     // keep CUDA's libm and four)
-    int max_acc = 8;  // (the emitter's own rule: Emitter::row_libm_on)
-    if (const char* e = getenv("RN_ROW_LIBM_MAX_ACC")) max_acc = atoi(e);
-    const bool row_libm = getenv("RN_ROW_LIBM") ? atoi(getenv("RN_ROW_LIBM")) != 0 : (!eo.mma && wpc_sizes(*P, eo).reg_accumulators <= max_acc);
-    eo.interleave = regs <= 128 ? (row_libm ? 2 : 4) : 8;
+    eo.interleave = regs <= 128 ? (wpc_sizes(*P, eo).row_functions ? 2 : 4) : 8;
     if (const char* e = getenv("RN_INTERLEAVE")) eo.interleave = std::max(1, atoi(e));
   }
   K->source = emit_source(*P, eo);
@@ -408,16 +404,8 @@ static int get_kernel(rn_model* m, const rn_config* cfg, Kernel** out, std::stri
 
   std::vector<const char*> opts = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo"};
   opts.push_back(key.fast ? "--fmad=true" : "--fmad=false");
-  if (getenv("RN_LIBM_NOINLINE")) opts.push_back("-DRN_LIBM_NOINLINE=1");
   const std::string block_def = "-DRN_BLOCK_DIM=" + std::to_string(key.block);
   if (key.block > 0) opts.push_back(block_def.c_str());
-  std::vector<std::string> extra_defs;  // experiment switches of the device sources (RN_X_*): RN_NVRTC_DEFS="-DRN_X_P_REGS=1 ..."
-  if (const char* e = getenv("RN_NVRTC_DEFS")) {
-    std::istringstream is(e);
-    std::string tok;
-    while (is >> tok) extra_defs.push_back(tok);
-    for (const std::string& t : extra_defs) opts.push_back(t.c_str());
-  }
   std::string maxreg;
   {
     // registers/thread: the fused iteration kernel is latency-bound on dependent fp64 chains, so occupancy matters

@@ -80,23 +80,9 @@ RN_DEVICE RnTs rn_ts_get() {
 #endif
 #define RN_TSD(slot) T.d[(unsigned)(slot) * T.bs]
 #define RN_TSI(slot) T.i[(unsigned)(slot) * T.bs]
-#ifndef RN_X_P_REGS
-#define RN_X_P_REGS 1 /* momentum in registers: 3.25 ms vs 3.41 ms per launch at the headline size with it in shared memory */
-#endif
-#ifndef RN_X_NORMALS
-/* flat rejection loop + second pass kept as a LOOP (the kernel is sensitive to code size: 3.41 vs 3.68 ms fully unrolled, round 2),
-   two pairs per trip since the second session of round 2: with the check-free division / square root and the one-branch log the two chains of a trip
-   overlap (2.505 -> 2.482 ms; the hand-paired form, RN_X_NORMALS == 4, is slower: 2.554 -- profiles/r2_sweep_iter_v4_*.jsonl) */
-#define RN_X_NORMALS 3
-#endif
-#define RN_Z(i) RN_TSD(RN_TS_P + (i)) /* scratch of the normal draws (aliases the shared-memory momentum) */
-#if RN_X_P_REGS
-#define RN_P(i) s.p[i]                /* experiment switch: momentum in registers */
-#else
-#define RN_P(i) RN_TSD(RN_TS_P + (i)) /* momentum in shared memory */
-#endif
+#define RN_Z(i) RN_TSD(RN_TS_P + (i)) /* scratch of the normal draws */
+#define RN_P(i) s.p[i] /* momentum in registers: 3.25 ms vs 3.41 ms per launch at the headline size with it in shared memory */
 #define RN_MASSD(i) RN_TSD(RN_TS_MASS + (i))
-#define RN_SNAP_P(i) RN_TSD(RN_TS_SNAP + (i))
 #define RN_ST_E_MEAN RN_TSD(RN_TS_STAT + 0)
 #define RN_ST_E_RAW RN_TSD(RN_TS_STAT + 1)
 #define RN_ST_TRANS2 RN_TSD(RN_TS_STAT + 2)
@@ -139,15 +125,13 @@ RN_DEVICE void rn_ring_add(const RnArgs& A, int c, const RnTs& T, int which, dou
   RN_STCS(&RN_AT(A.st_rings, which * A.stats_window + i, c), value);
 }
 
-struct RnPQ {  // pqBuf's q and potential + the gradient at pqBuf.q  (pqBuf's p: RN_P, shared memory)
+struct RnPQ {  // pqBuf's q, p and potential + the gradient at pqBuf.q
   double q[RN_N], g[RN_N];
   double U;
-#if RN_X_P_REGS
   double p[RN_N];
-#endif
 };
 
-// velocity_i = (M^-1 p)_i  (LeapFrog.scala:205-219); p is the shared-memory momentum
+// velocity_i = (M^-1 p)_i  (LeapFrog.scala:205-219)
 RN_DEVICE double rn_velocity_i(const RnArgs& A, int c, const RnTs& T, const RnPQ& s, int kind, int i) {
   (void)s;
   (void)T;
@@ -236,10 +220,6 @@ RN_DEVICE void rn_take_steps(const RnArgs& A, int c, const RnTs& T, int kind, Rn
 // of the per-pair maxima), and a second, convergent pass applies sqrt(-2 log(s)/s).  s is recomputed there from the
 // parked v1, v2 by the same two products and one sum -> the same bits.
 RN_DEVICE void rn_draw_normals(const RnTs& T, RnRng& rng) {
-#if RN_X_NORMALS == 2
-  for (int i = 0; i < RN_N; i++) RN_Z(i) = rn_normal(rng);  // experiment switch: one nextGaussian at a time
-  return;
-#endif
   int i0 = 0;
   if (rng.have) {
     rng.have = 0;
@@ -247,11 +227,8 @@ RN_DEVICE void rn_draw_normals(const RnTs& T, RnRng& rng) {
     i0 = 1;
   }
   const int npairs = (RN_N - i0 + 1) / 2;  // the last pair's second variate may be left over (-> rng.nng); slot RN_N is scratch
-#ifndef RN_X_POLAR2
-#define RN_X_POLAR2 1 /* 2.488 -> 2.467 ms per launch at the headline size (profiles/r2_sweep_iter_v6_polar2_merged.jsonl) */
-#endif
-#if RN_X_POLAR2
-  // two attempts per trip (see rn_polar_attempt2); the second one is consumed only if it is needed
+  // two attempts per trip (see rn_polar_attempt2); the second one is consumed only if it is needed: 2.488 -> 2.467 ms per launch
+  // at the headline size (profiles/r2_sweep_iter_v6_polar2_merged.jsonl)
   for (int k = 0; k < npairs;) {
     double a1, a2, b1, b2;
     rn_i64 seed4, seed8;
@@ -272,56 +249,11 @@ RN_DEVICE void rn_draw_normals(const RnTs& T, RnRng& rng) {
     rng.seed = needb ? seed8 : seed4;
     k = kb + (okb ? 1 : 0);
   }
-#else
-  for (int k = 0; k < npairs;) {
-    double v1, v2;
-    rn_polar_attempt(rng, v1, v2);
-    const double s = v1 * v1 + v2 * v2;
-    if (!(s >= 1 || s == 0)) {
-      RN_Z(i0 + 2 * k) = v1;
-      RN_Z(i0 + 2 * k + 1) = v2;
-      k += 1;
-    }
-  }
-#endif
-#if RN_X_NORMALS == 4 && RN_X_SPEC && !defined(RN_FAST_MATH) && !(defined(RN_X_LIBM_PLAIN) && RN_X_LIBM_PLAIN)
-  // two pairs per trip: their log -> division -> square root chains are independent, and with the `_try` form of the log (one
-  // shared fallback branch) they sit in ONE basic block, so ptxas interleaves them.  An odd number of pairs repeats the last
-  // pair (same inputs, same outputs, written twice).
-#pragma unroll 1
-  for (int k = 0; k < npairs; k += 2) {
-    const int ia = i0 + 2 * k, ib = i0 + 2 * (k + 1 < npairs ? k + 1 : k);
-    const double a1 = RN_Z(ia), a2 = RN_Z(ia + 1), b1 = RN_Z(ib), b2 = RN_Z(ib + 1);
-    const double sa = a1 * a1 + a2 * a2, sb = b1 * b1 + b2 * b2;
-    bool oka, okb;
-    double la = rn_strict_log_try(sa, oka), lb = rn_strict_log_try(sb, okb);
-    if (!(oka && okb)) {
-      la = rn_strict_log_full(sa);
-      lb = rn_strict_log_full(sb);
-    }
-    const double ma = rn_sqrt_nc(rn_div_nc(-2 * la, sa)), mb = rn_sqrt_nc(rn_div_nc(-2 * lb, sb));  // ranges: rn_polar_multiplier
-    RN_Z(ia) = a1 * ma;
-    if (ia + 1 < RN_N) {
-      RN_Z(ia + 1) = a2 * ma;
-    } else {
-      rng.nng = a2 * ma;
-      rng.have = 1;
-    }
-    RN_Z(ib) = b1 * mb;
-    if (ib + 1 < RN_N) {
-      RN_Z(ib + 1) = b2 * mb;
-    } else {
-      rng.nng = b2 * mb;
-      rng.have = 1;
-    }
-  }
-  return;
-#endif
-#if RN_X_NORMALS == 1
-#pragma unroll 1
-#elif RN_X_NORMALS == 3
+  // the second pass kept as a loop (the kernel is sensitive to code size: 3.41 vs 3.68 ms fully unrolled, round 2), two pairs per
+  // trip: with the check-free division / square root and the one-branch log the two chains of a trip overlap (2.505 -> 2.482 ms;
+  // a hand-paired form through rn_strict_log_try, sharing one fallback branch, was slower: 2.554 --
+  // profiles/r2_sweep_iter_v4_nocheck_div_spec_kconst.jsonl)
 #pragma unroll 2
-#endif
   for (int k = 0; k < npairs; k++) {
     const int i = i0 + 2 * k;
     const double v1 = RN_Z(i), v2 = RN_Z(i + 1);
@@ -344,10 +276,8 @@ RN_DEVICE void rn_initialize_ps(const RnArgs& A, int c, const RnTs& T, RnPQ& s, 
   (void)kind;
   (void)s;
   rn_draw_normals(T, rng);  // buf(i) = rng.standardNormal
-#if RN_X_P_REGS
   RN_UNROLL
   for (int i = 0; i < RN_N; i++) s.p[i] = RN_Z(i);
-#endif
 #if RN_MASS_MAX >= 2
   if (kind == 2) {  // DenseMassMatrix.upperTriangularSolve, MassMatrix.scala:55-72; in place: slot i holds z_i until p_i
     int i = RN_N - 1;  // replaces it, and p_i only reads z_i and the p_j, j > i, already in place
@@ -364,9 +294,7 @@ RN_DEVICE void rn_initialize_ps(const RnArgs& A, int c, const RnTs& T, RnPQ& s, 
       i -= 1;
       m -= 1;
     }
-#if RN_X_P_REGS
     for (int k = 0; k < RN_N; k++) s.p[k] = RN_Z(k);
-#endif
     return;
   }
 #endif
@@ -552,32 +480,23 @@ RN_DEVICE void rn_iterate(const RnArgs& A) {
   // was replaced in between.  It is carried in a register and recomputed only then (and at the start of a launch).
   bool havePrevH = false;
 
-  // RN_X_KEEP_STATE: the current position, its gradient and potential stay in registers from one iteration to the next -- after an
+  // The current position, its gradient and potential stay in registers from one iteration to the next -- after an
   // accepted proposal they ARE the state the next iteration starts from, so only a rejection re-reads them from `params` (which is
   // written on accept exactly as before: it is what a rejection restores, what isUTurn measures against, and the state the launch
   // leaves behind).  The drawn momentum reaches `params` only where the reference's copy survives the iteration: on rejection
-  // (from the scratch of the normal draws, intact while the momentum lives in registers under the identity mass).
-#ifndef RN_X_KEEP_STATE
-#define RN_X_KEEP_STATE 1 /* with the compile-time CTA size: 2.446 -> 2.400 ms per launch (profiles/r2_sweep_iter_v7_keep_state_block_dim.jsonl) */
-#endif
-#define RN_KEEP_P_LATE (RN_X_KEEP_STATE && RN_X_P_REGS)
+  // (from the scratch of the normal draws, intact while the momentum lives in registers under the identity mass).  With the
+  // compile-time CTA size: 2.446 -> 2.400 ms per launch (profiles/r2_sweep_iter_v7_keep_state_block_dim.jsonl).
   RnPQ s;
-#if RN_X_KEEP_STATE
   RN_UNROLL
   for (int i = 0; i < RN_N; i++) {
     s.q[i] = RN_AT(A.params, RN_N + i, c);
     s.g[i] = RN_AT(A.grad, i, c);
   }
   s.U = RN_AT(A.params, 2 * RN_N, c);
-#endif
 
   for (int it = 0; it < A.n_iter; it++) {
     // ---------------- lf.startIteration, LeapFrog.scala:52-59 ----------------
-#if RN_X_KEEP_STATE
     const double cU = s.U;
-#else
-    const double cU = RN_AT(A.params, 2 * RN_N, c);
-#endif
     if (!havePrevH) {
       RN_UNROLL
       for (int i = 0; i < RN_N; i++) RN_P(i) = RN_AT(A.params, i, c);  // old momentum
@@ -588,19 +507,10 @@ RN_DEVICE void rn_iterate(const RnArgs& A) {
       rn_initialize_ps(A, c, T, s, kind, rng);
       rn_rng_park(T, rng);
     }
-#if RN_X_KEEP_STATE
-    if (!(RN_KEEP_P_LATE && kind == 0)) {
+    if (kind != 0) {  // initializePs writes into params (LeapFrog.scala:55); identity mass: on rejection only, below
       RN_UNROLL
       for (int i = 0; i < RN_N; i++) RN_AT(A.params, i, c) = RN_P(i);
     }
-#else
-    RN_UNROLL
-    for (int i = 0; i < RN_N; i++) {
-      RN_AT(A.params, i, c) = RN_P(i);  // initializePs writes into params (LeapFrog.scala:55); kept on reject
-      s.q[i] = RN_AT(A.params, RN_N + i, c);
-      s.g[i] = RN_AT(A.grad, i, c);
-    }
-#endif
     s.U = cU;
     RN_TS_START_H = rn_energy(A, c, T, s, kind, cU);  // finishIteration's energy(params), :62
     const double usedStep = stepSize;
@@ -631,20 +541,12 @@ RN_DEVICE void rn_iterate(const RnArgs& A) {
           rn_take_steps(A, c, T, kind, s, 1, stepSize, S);
           if (l == A.min_steps) {
             snap = s;
-#if !(RN_X_P_REGS)
-            RN_UNROLL
-            for (int i = 0; i < RN_N; i++) RN_SNAP_P(i) = RN_P(i);
-#endif
           }
         }
         if (l < A.min_steps) {
           rn_take_steps(A, c, T, kind, s, A.min_steps - l, stepSize, S);
         } else {
           s = snap;
-#if !(RN_X_P_REGS)
-          RN_UNROLL
-          for (int i = 0; i < RN_N; i++) RN_P(i) = RN_SNAP_P(i);
-#endif
         }
         // steps.add(l), Stats.scala:24-30
         ring_i += 1;
@@ -686,15 +588,13 @@ RN_DEVICE void rn_iterate(const RnArgs& A) {
     } else {
       RN_UNROLL
       for (int i = 0; i < RN_N; i++) s.q[i] = RN_AT(A.params, RN_N + i, c);  // s.q := current position either way
-#if RN_X_KEEP_STATE
       RN_UNROLL
       for (int i = 0; i < RN_N; i++) s.g[i] = RN_AT(A.grad, i, c);
       s.U = RN_AT(A.params, 2 * RN_N, c);
-      if (RN_KEEP_P_LATE && kind == 0) {  // the momentum drawn at startIteration stays in params (LeapFrog.scala:55)
+      if (kind == 0) {  // the momentum drawn at startIteration stays in params (LeapFrog.scala:55)
         RN_UNROLL
         for (int i = 0; i < RN_N; i++) RN_AT(A.params, i, c) = RN_Z(i);
       }
-#endif
       eH = startH;
     }
     {  // stats.energyVariance.update(eH); energyTransitions2 += pow(eH - prevH, 2)

@@ -11,7 +11,7 @@ C_, I_ = 151552, 100
 rir = open(os.path.join(ROOT, "rainier_b200", "models", sys.argv[1] if len(sys.argv) > 1 else "funnel10.rir"), "rb").read()
 caps = [int(x) for x in os.environ.get("SWEEP_CAPS", "128,96").split(",")]
 blocks = [int(x) for x in os.environ.get("SWEEP_BLOCKS", "128").split(",")]
-defsets = os.environ.get("SWEEP_DEFS", "|-DRN_X_LIBM_PLAIN=1 -DRN_X_LIBM_FULL_INLINE=1|-DRN_X_LIBM_FULL_INLINE=1|-DRN_X_P_REGS=0|-DRN_X_NORMALS=0|-DRN_X_NORMALS=2").split("|")
+defsets = os.environ.get("SWEEP_DEFS", "").split("|")
 math = abi.RN_MATH_FAST if os.environ.get("SWEEP_FAST") else abi.RN_MATH_PARITY
 ref = None
 for defs in defsets:
@@ -21,7 +21,6 @@ for defs in defsets:
         for tok in defs.split():
             if tok.startswith("ENV:"):
                 os.environ[tok[4:].split("=")[0]] = tok.split("=", 1)[1]
-        os.environ["RN_NVRTC_DEFS"] = " ".join(t for t in defs.split() if not t.startswith("ENV:"))
         os.environ["RN_MAXRREGCOUNT"] = str(cap)
         os.environ["RN_BLOCK"] = str(block)
         model = api.CudaModel(rir, [], device=0)

@@ -11,7 +11,6 @@ rir = open(os.path.join(ROOT, "rainier_b200", "models", "funnel10.rir"), "rb").r
 cfg = api.make_config(iterations=100, warmupIterations=0, sampler=api.HMCSampler(5), stepSizeTuner=api.StaticStepSize(0.1),
                       massMatrixTuner=api.IdentityMassMatrixTuner(), launchIterations=100)
 for defs in (sys.argv[1:] or [""]):
-    os.environ["RN_NVRTC_DEFS"] = defs
     m = api.CudaModel(rir, [], device=-1)
     cub = "/tmp/sass_iter.cubin"
     open(cub, "wb").write(m.emit_cubin(cfg))

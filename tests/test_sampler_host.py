@@ -12,13 +12,13 @@ from rainier_b200 import abi, api
 import host_emulation as he
 
 
-def _run(model, config, seeds, dense=False, defs=""):
+def _run(model, config, seeds, dense=False):
     rir, cols = model.compile(True)
     cfg, keep = api.lower_config(config)
     cfg.backend = abi.RN_BACKEND_THREAD
     cm = api.CudaModel(rir, cols, device=-1)
     config.backend = abi.RN_BACKEND_THREAD
-    got = he.sample(defs + cm.emit_source(config), cfg, seeds, cm)
+    got = he.sample(cm.emit_source(config), cfg, seeds, cm)
     ref = OracleModel(rir, cols).sample(cfg, seeds=seeds, trace=True, dense_mass=dense)
     assert np.array_equal(got["trace"][:, :, 1], ref["trace"][:, :, 1]), "accept decisions differ"
     assert np.array_equal(got["trace"][:, :, 3], ref["trace"][:, :, 3]), "leapfrog step counts differ"
@@ -38,16 +38,15 @@ def test_hmc_dualavg_funnel_on_host():
     _run(configs.funnel(), _cfg(30, 120, api.HMCSampler(5), api.DualAvgTuner(0.8), api.IdentityMassMatrixTuner()), np.arange(6) + 7)
 
 
-@pytest.mark.parametrize("defs", ["#define RN_X_NORMALS 4\n", "#define RN_X_SPEC 0\n", "#define RN_X_KCONST 0\n#define RN_X_NORMALS 1\n", "#define RN_X_POLAR2 0\n", "#define RN_X_KEEP_STATE 0\n"])
-def test_round2b_source_variants_on_host(defs):
-    """the experiment switches of round 2b (two polar pairs per trip through the `_try` form of the log; the branching forms of
-    the fdlibm common paths; coefficients as literals) leave every bit where it was -- even and odd numbers of parameters
-    (odd: the cached second variate alternates, the last pair of a draw is repeated by the two-at-a-time pass)"""
-    _run(configs.funnel(), _cfg(12, 40, api.HMCSampler(5), api.DualAvgTuner(0.8), api.IdentityMassMatrixTuner()), np.arange(4) + 7, defs=defs)
-    _run(configs.funnel(7), _cfg(12, 30, api.HMCSampler(4), api.DualAvgTuner(0.8), api.IdentityMassMatrixTuner()), np.arange(3) + 3, defs=defs)
+def test_round2b_source_variants_on_host():
+    """the round-2b forms of the sampler source (two polar attempts and two second-pass pairs per trip, speculative fdlibm common
+    paths with their coefficients in the constant bank, state kept in registers across iterations) are bit-exact -- even and odd
+    numbers of parameters (odd: the cached second variate alternates)"""
+    _run(configs.funnel(), _cfg(12, 40, api.HMCSampler(5), api.DualAvgTuner(0.8), api.IdentityMassMatrixTuner()), np.arange(4) + 7)
+    _run(configs.funnel(7), _cfg(12, 30, api.HMCSampler(4), api.DualAvgTuner(0.8), api.IdentityMassMatrixTuner()), np.arange(3) + 3)
     model = sbc_models.build("SBCGamma")[0]
-    _run(model, _cfg(10, 30, api.HMCSampler(3), api.DualAvgTuner(0.8), api.IdentityMassMatrixTuner()), np.arange(3) + 2, defs=defs)
-    _run(configs.eight_schools(), api.SamplerConfig(iterations=10, warmupIterations=60), np.arange(2) + 11, defs=defs)
+    _run(model, _cfg(10, 30, api.HMCSampler(3), api.DualAvgTuner(0.8), api.IdentityMassMatrixTuner()), np.arange(3) + 2)
+    _run(configs.eight_schools(), api.SamplerConfig(iterations=10, warmupIterations=60), np.arange(2) + 11)
 
 
 def test_default_config_eight_schools_on_host():
@@ -238,40 +237,18 @@ def test_wpc_rerolled_invariant_sections_on_host():
     _run_wpc(model, cfg, np.arange(2) + 9, tol=1e-9, rir_gpu=prir, cols_gpu=pcols, tma="2", k="2", chains_per_cta=2)
 
 
-@pytest.mark.parametrize("switch", ["RN_ROW_FUSED_SWEEPS", "RN_SCATTER_REUSE_INDEX", "RN_ROW_LIBM"])
-def test_wpc_opt_in_emitter_switches_on_host(switch, monkeypatch):
-    """the measured-and-rejected variants of the warp-per-chain row bodies stay correct while they stay in the tree: a group's
-    reverse statements right after its forward statements (the row's fold additions recognised as joiners, no second read of the
-    tile), the forward Lookup's index reused by the scatter-add, CUDA's libm instead of the row functions -- same accept decisions
-    as the oracle, densities to the tolerance of this shape, on a Lookup / scatter model and on a regression with dot products"""
-    monkeypatch.setenv(switch, "0" if switch == "RN_ROW_LIBM" else "1")
-    model = configs.poisson_glm(48, 768)
+def test_wpc_row_bodies_with_cuda_libm_on_host(monkeypatch):
+    """row bodies that keep more than 8 accumulators in registers use CUDA's exp / log instead of the branch-free row functions
+    (rn_emit.cpp: row_functions): the rows-across-lanes logistic regression with 8 covariates (9 accumulators) and no DMMA path -- same accept
+    decisions as the oracle, densities to the tolerance of this shape"""
+    monkeypatch.setenv("RN_MMA", "0")
+    model = configs.logreg(600, 8)  # 75 rows of 8 observations: data tiles with two warps per chain as well
     prir, pcols = model.compile(False)
-    cfg = api.make_config(iterations=4, warmupIterations=0, sampler=api.HMCSampler(3), stepSizeTuner=api.StaticStepSize(0.004),
+    cfg = api.make_config(iterations=5, warmupIterations=0, sampler=api.HMCSampler(3), stepSizeTuner=api.StaticStepSize(0.02),
                           massMatrixTuner=api.IdentityMassMatrixTuner())
     cfg.backend = abi.RN_BACKEND_WARP
     src = api.CudaModel(prir, pcols, device=-1).emit_source(cfg)
     dens = src[src.index("// ---- emitted"):src.index("// rn_sampler_wpc.cuh --")]
-    if switch == "RN_ROW_FUSED_SWEEPS":
-        assert "RN_FENCE();" not in dens[dens.index("// target 1"):]
-    if switch == "RN_SCATTER_REUSE_INDEX":
-        assert "rn_tab_lookup_k(" in dens[dens.index("// target 1"):]
-    if switch == "RN_ROW_LIBM":
-        assert "rn_row_exp(" not in dens and " exp(" in dens
+    assert " exp(" in dens and " log(" in dens and "rn_row_" not in dens
     _run_wpc(model, cfg, np.arange(2) + 9, tol=1e-9, rir_gpu=prir, cols_gpu=pcols, tma="2")
     _run_wpc(model, cfg, np.arange(2) + 9, tol=1e-9, rir_gpu=prir, cols_gpu=pcols, tma="2", k="2", chains_per_cta=2)
-    model = configs.logreg(300, 3)
-    prir, pcols = model.compile(False)
-    cfg = api.make_config(iterations=5, warmupIterations=0, sampler=api.HMCSampler(3), stepSizeTuner=api.StaticStepSize(0.02),
-                          massMatrixTuner=api.IdentityMassMatrixTuner())
-    monkeypatch.setenv("RN_MMA", "0")
-    _run_wpc(model, cfg, np.arange(2) + 9, tol=1e-9, rir_gpu=prir, cols_gpu=pcols, tma="2")
-
-
-def test_merged_fallback_density_on_host(monkeypatch):
-    """RN_MERGED_FALLBACK (opt-in, measured slower): the fdlibm calls of a data-free density share one fallback branch; the
-    complete functions re-evaluate the density when any argument left a common path -- bit-identical to the oracle through an
-    adaptive warmup (whose step-size search doubles the step until the trajectory leaves the common paths' domain)"""
-    monkeypatch.setenv("RN_MERGED_FALLBACK", "1")
-    _run(configs.funnel(), _cfg(12, 40, api.HMCSampler(5), api.DualAvgTuner(0.8), api.IdentityMassMatrixTuner()), np.arange(4) + 7)
-    _run(configs.eight_schools(), api.SamplerConfig(iterations=10, warmupIterations=60), np.arange(2) + 11)
